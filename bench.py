@@ -13,6 +13,10 @@ e2e    = the same metric through the C-ABI with HOST buffers: state + factors H2
 N > 1  = N independent replicas (one window per GPU, no data-path collective; "weak"); the
          landmark-sharded C4 run with its NCCL all-reduce is reported under "c4".
 One JSON line on stdout (rank 0).
+--dump-outputs DIR writes what the last timed solve returned to its caller (rank 0) as DIR/<name>.npy in float64:
+the state read back after it (control points, biases, inverse depths, line delay) and its summary, and the same for
+the last e2e step under the prefix "e2e_".  The inputs are seeded, so two builds run with the same arguments can be
+compared array for array.
 """
 import argparse
 import importlib
@@ -134,6 +138,20 @@ def oracle_lib():
     if not os.path.exists(so):
         subprocess.run(["make", "-C", os.path.join(ROOT, "oracle")], check=True, capture_output=True)
     return pkg.CtvioLib(so, "ctvo_", optional=pkg.binding.DEVICE_ONLY_SYMBOLS)
+
+
+def solve_outputs(prefix, summary, q, p, biases, inv_depths, line_delay):
+    """What a caller of solve receives: the summary and the state read back after it."""
+    return {prefix + "knots_q": q, prefix + "knots_p": p, prefix + "biases": biases, prefix + "inv_depths": inv_depths,
+            prefix + "line_delay": [line_delay], prefix + "cost": [summary.initial_cost, summary.final_cost],
+            prefix + "lm_steps": [summary.iterations, summary.num_successful_steps, summary.num_unsuccessful_steps,
+                                  summary.termination, summary.num_jacobian_evals]}
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def cpu_solve_rate(w, threads, budget_s):
@@ -411,6 +429,9 @@ def run_reference(args, rank, world):
             per_step.append(dt)
             evals += w.n_residual_blocks * s.num_jacobian_evals
             iters += s.iterations
+    if args.dump_outputs:
+        q, p = est.GetKnots()
+        dump_outputs(args.dump_outputs, solve_outputs("", s, q, p, est.GetBiases(), est.GetInvDepths(), est.GetLineDelay()))
     total = sum(per_step)
     value = evals / total
     line = {
@@ -441,6 +462,7 @@ def main():
     ap.add_argument("--impl", default="ctvio", choices=["ctvio", "reference"])
     ap.add_argument("--cpu-budget-s", type=float, default=10.0)
     ap.add_argument("--no-c4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ctvio" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
@@ -503,6 +525,9 @@ def main():
     clocks = sampler.stop()
     dev_s = sum(per_ms) * 1e-3
     summ = s
+    if args.dump_outputs and rank == 0:
+        q, p = est.GetKnots()
+        outputs = solve_outputs("", s, q, p, est.GetBiases(), est.GetInvDepths(), est.GetLineDelay())
 
     # ---------------- e2e path: host buffers through the C-ABI ----------------
     e2e_est = pkg.Estimator(lib, pkg.make_config(device=local_rank, **w.config_kwargs()))
@@ -530,6 +555,9 @@ def main():
             e2e_evals += n_blocks * s2.num_jacobian_evals
     barrier()
     e2e_s = sum(e2e_times)
+    if args.dump_outputs and rank == 0:
+        outputs.update(solve_outputs("e2e_", s2, q, p, b, r, ld))
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---------------- kernel stage timings + roofline of the dominant kernel ----------------
     prof = est.ProfileKernels(reps=20, flush_l2=True) if rank == 0 else None
